@@ -237,6 +237,42 @@ def bits_equal(a, b):
         a.numel() == 0 or torch.equal(a.contiguous().view(-1).view(torch.uint8), b.contiguous().view(-1).view(torch.uint8)))
 
 
+DUMP_SAMPLE = 8192  # elements kept per tensor: 1455 tensors x 8192 x 4 B = 48 MB, within the 64 MB a dump may take
+
+
+def dump_outputs(path, out_dir):
+    """Writes the checkpoint file ``path``, as ``torch.load`` returns it, to ``out_dir/<key path>.npy`` (e.g.
+    ``optimizer.state.0.exp_avg.npy``), flattened, as float32 (float64 stays float64).  A tensor of more than DUMP_SAMPLE
+    elements is sampled: its first 16 elements (the narrowing edge values sit there) and the rest at positions drawn with a fixed
+    seed, so two builds run with the same arguments write the same positions.  Every value written is finite: a non-finite
+    element (the workload holds +-inf and NaN on purpose) is written as 0, and ``<key path>.nonfinite.npy`` beside it says
+    which ones it replaced (same positions: 0 finite, 1 +inf, -1 -inf, 2 NaN); tensors without any get no such file."""
+    import numpy as np
+
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    rng = np.random.default_rng(0)
+    loaded = torch.load(path, weights_only=False, mmap=True)
+
+    def walk(x, prefix):
+        for k, v in (x.items() if isinstance(x, dict) else enumerate(x)):
+            if isinstance(v, (dict, list, tuple)):
+                walk(v, f"{prefix}{k}.")
+            elif isinstance(v, torch.Tensor):
+                flat = v.reshape(-1)
+                if flat.numel() > DUMP_SAMPLE:
+                    rest = rng.choice(flat.numel() - 16, DUMP_SAMPLE - 16, replace=False) + 16
+                    flat = flat[torch.from_numpy(np.concatenate([np.arange(16), np.sort(rest)]))]
+                values = (flat if flat.dtype == torch.float64 else flat.float()).numpy()
+                if not np.isfinite(values).all():
+                    kind = np.isposinf(values) * 1.0 - np.isneginf(values) + np.isnan(values) * 2.0
+                    np.save(out_dir / f"{prefix}{k}.nonfinite.npy", kind.astype(values.dtype))
+                    values = np.where(np.isfinite(values), values, 0).astype(values.dtype)
+                np.save(out_dir / f"{prefix}{k}.npy", values)
+
+    walk(loaded, "")
+
+
 # ----------------------------------------------------------------------------------------------------
 # the two arms behind one interface
 # ----------------------------------------------------------------------------------------------------
@@ -616,6 +652,8 @@ def run_arm(args, rank, world, local):
             ok &= bits_equal(a, b.to(torch.bfloat16).cpu() if narrowed else b.cpu())
         check = "bit-exact" if ok else "MISMATCH"
         del loaded, lt
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(path, args.dump_outputs)
 
     load_ms = base_ms = None
     if not args.no_training_loop:
@@ -767,7 +805,11 @@ def main():
     ap.add_argument("--no-ceiling", action="store_true")
     ap.add_argument("--no-c3-kernel", action="store_true", help="skip the C3 (narrowing) kernel-only leg of the default run")
     ap.add_argument("--traffic-bytes", type=float, default=None, help="dram read+write bytes per launch from the ncu capture")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write rank 0's checkpoint of the last step to DIR/<key path>.npy (sampled, see dump_outputs)")
     args, rest = ap.parse_known_args()
+    if args.dump_outputs and args.config == "c4":
+        raise SystemExit("--dump-outputs covers the configs c2 and c3")
     if args.narrow:
         args.config = "c3"
     args.narrow = args.config == "c3"

@@ -12,8 +12,12 @@ def _outcome(fn):
         return {"raises": type(exc).__name__, "message": _scrub(str(exc))}
 
 
+_TMP_ROOTS = []  # the directories scenarios() was given: a temporary directory need not live under /tmp
+
+
 def _scrub(text):
-    text = re.sub(r"/tmp/[^\s'\"]+|/dev/shm/[^\s'\"]+", "<path>", text)
+    roots = "".join(re.escape(r) + r"[^\s'\"]*|" for r in _TMP_ROOTS)
+    text = re.sub(roots + r"/tmp/[^\s'\"]+|/dev/shm/[^\s'\"]+", "<path>", text)
     return re.sub(r"0x[0-9a-f]+", "<addr>", text)
 
 
@@ -49,6 +53,7 @@ def scenarios(tmp):
     from nvidia_resiliency_ext.checkpointing.local.ckpt_managers.local_manager import LocalCheckpointManager
     from nvidia_resiliency_ext.checkpointing.local.replication.group_utils import parse_group_sequence
 
+    _TMP_ROOTS[:] = [os.path.realpath(tmp), os.path.abspath(tmp)]
     out = {}
     counter = [0]
 

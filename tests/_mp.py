@@ -34,8 +34,20 @@ def run_ranks(fn, world: int, *args, backend: str = "gloo", timeout: float = 150
     errq = ctx.SimpleQueue()
     port = free_port()
     procs = [ctx.Process(target=_entry, args=(r, world, port, backend, fn, args, errq)) for r in range(world)]
-    for p in procs:
-        p.start()
+    # gloo ranks run the host-only paths: they must not see this machine's GPUs, or they would take the device paths, whose
+    # point-to-point payloads gloo cannot send.  The children inherit the environment at start.
+    hidden = os.environ.get("CUDA_VISIBLE_DEVICES")
+    if backend == "gloo":
+        os.environ["CUDA_VISIBLE_DEVICES"] = ""
+    try:
+        for p in procs:
+            p.start()
+    finally:
+        if backend == "gloo":
+            if hidden is None:
+                del os.environ["CUDA_VISIBLE_DEVICES"]
+            else:
+                os.environ["CUDA_VISIBLE_DEVICES"] = hidden
     for p in procs:
         p.join(timeout)
     errors = []

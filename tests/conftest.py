@@ -71,21 +71,25 @@ def built_library():
     return path
 
 
-@pytest.fixture(scope="session")
-def dist_1rank():
-    """A world of one rank (gloo on CPU boxes, NCCL when a GPU is present) for the collective-by-contract APIs."""
+@pytest.fixture
+def dist_1rank(request):
+    """A world of one rank for the collective-by-contract APIs: NCCL for tests marked ``gpu`` on a machine with a GPU, gloo
+    for all others, so that a CPU test sees the same process group with or without a GPU (the stand-in device's tensors are
+    host memory, which NCCL refuses).  Kept for the session; re-created only when the next test needs the other backend."""
     import torch
     import torch.distributed as dist
 
+    backend = "nccl" if request.node.get_closest_marker("gpu") and torch.cuda.is_available() else "gloo"
+    if dist.is_initialized() and dist.get_backend() != backend:
+        dist.destroy_process_group()
     if not dist.is_initialized():
         os.environ["MASTER_ADDR"] = "127.0.0.1"
         os.environ["MASTER_PORT"] = str(free_port())
-        backend = "nccl" if torch.cuda.is_available() else "gloo"
         if backend == "nccl":
             torch.cuda.set_device(0)
         dist.init_process_group(backend, rank=0, world_size=1)
     yield
-    # left initialised for the whole session; pytest exits the process afterwards
+    # left initialised; pytest exits the process afterwards
 
 
 @pytest.fixture

@@ -99,7 +99,7 @@ def _args(B, **over):
 
     ns = argparse.Namespace(gpus=1, steps=2, warmup=3, impl="engine", config="c2", narrow=False, persist_steps=1, load_reps=1, scale=1.0,
                             baseline_sample_gb=0.001, no_cpu_baseline=True, no_verify=False, no_restore=False, no_training_loop=True,
-                            no_ceiling=True, no_c3_kernel=False, traffic_bytes=None)
+                            no_ceiling=True, no_c3_kernel=False, traffic_bytes=None, dump_outputs=None)
     for k, v in over.items():
         setattr(ns, k, v)
     return ns
@@ -134,6 +134,39 @@ def test_run_arm_assembles_the_same_config_in_both_arms(bench, monkeypatch, buil
     assert eng["roofline"]["bound"] == "hbm" and eng["roofline"]["algorithmic_bytes_per_launch"] > 0 and "roofline" not in ref and "cpu_baseline" in ref
     assert "error" not in eng["c3_kernel_roofline"] and eng["c3_kernel_roofline"]["algorithmic_bytes_per_launch"] > 0 and "c3_kernel_roofline" not in c3
     assert eng["restore_verify"] == "bit-exact" and c3["config"]["workload"] == B.WORKLOADS["c3"] and c3["dtype"].startswith("f32->bf16")
+
+
+def test_dump_outputs_writes_the_last_checkpoint(bench, monkeypatch, built_library, dist_1rank, tmp_path):
+    """--dump-outputs: run_arm writes the checkpoint of its last timed step as float32 .npy files named by key path, whole
+    when small, else the first 16 elements plus a seeded sample at the same positions in every run; non-finite elements are
+    written as 0 and recorded in a .nonfinite.npy beside them."""
+    import numpy as np
+
+    B = bench
+    monkeypatch.setattr(B, "ClockSampler", lambda idx: types.SimpleNamespace(__enter__=lambda: None, __exit__=lambda *a: None, summary=lambda: {"sm_mhz": None}))
+    with fake_device(monkeypatch) as (engine, lib):
+        monkeypatch.setattr(B, "llama3_8b_shard_state", lambda dev, seed=0, scale=1.0: (_small_state(), sum(t.numel() * t.element_size() for t in B.flatten(_small_state()))))
+        B.run_arm(_args(B, config="c3", narrow=True, no_restore=True, no_c3_kernel=True, dump_outputs=str(tmp_path / "c3")), 0, 1, 0)
+    sd = _small_state(fake=False)
+    names = {f"model.l{i}" for i in range(4)} | {f"optimizer.state.{i}.{k}" for i in range(4) for k in ("exp_avg", "step")}
+    assert {p.stem for p in (tmp_path / "c3").iterdir()} == names
+    got = np.load(tmp_path / "c3" / "model.l2.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, sd["model"]["l2"].to(torch.bfloat16).float().reshape(-1).numpy())
+
+    big = {"w": torch.randn(5000, generator=torch.Generator().manual_seed(1), dtype=torch.float64), "h": torch.arange(300, dtype=torch.bfloat16)}
+    big["w"][1:4] = torch.tensor([float("inf"), float("-inf"), float("nan")], dtype=torch.float64)
+    torch.save(big, tmp_path / "big.pt")
+    monkeypatch.setattr(B, "DUMP_SAMPLE", 100)
+    for run in ("a", "b"):
+        B.dump_outputs(tmp_path / "big.pt", tmp_path / run)
+    w, h = np.load(tmp_path / "a" / "w.npy"), np.load(tmp_path / "a" / "h.npy")
+    kind = np.load(tmp_path / "a" / "w.nonfinite.npy")
+    assert sorted(p.name for p in (tmp_path / "a").iterdir()) == ["h.npy", "w.nonfinite.npy", "w.npy"]
+    assert w.dtype == kind.dtype == np.float64 and w.shape == kind.shape == (100,) and np.array_equal(w, np.load(tmp_path / "b" / "w.npy"))
+    assert np.isfinite(w).all() and list(w[1:4]) == [0, 0, 0] and list(kind[:5]) == [0, 1, -1, 2, 0] and not kind[4:].any()
+    finite = big["w"].numpy()[np.isfinite(big["w"].numpy())]
+    assert w[0] == big["w"][0] and np.array_equal(w[4:16], big["w"][4:16].numpy()) and np.isin(w[4:], finite).all() and len(np.unique(w[4:])) == 96
+    assert h.dtype == np.float32 and h.shape == (100,) and np.array_equal(h[:16], np.arange(16))
 
 
 def test_d2h_ceiling_control_flow(bench, monkeypatch, dist_1rank):

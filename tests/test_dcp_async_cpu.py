@@ -193,7 +193,9 @@ def test_writer_process_reads_cuda_items_from_the_snapshot_slot(tmp_path, built_
 
     state = _state()
     sync_dir, async_dir = tmp_path / "sync", tmp_path / "async"
-    dcp.save(state, storage_writer=FileSystemWriter(sync_dir, thread_count=1), planner=DefaultSavePlanner())
+    # per_thread_copy_ahead=0: with one thread and a CUDA device present, PyTorch's writer would switch to its copy-ahead
+    # loader, which writes the items in order of size; the writer process never copies ahead (its items are on the host)
+    dcp.save(state, storage_writer=FileSystemWriter(sync_dir, thread_count=1, per_thread_copy_ahead=0), planner=DefaultSavePlanner())
 
     writer = FileSystemWriterAsync(async_dir, thread_count=1)
     _, metadata, dist_wrapper = save_state_dict_async_plan(state, writer, None, 0)
